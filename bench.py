@@ -3,6 +3,7 @@
 
   python bench.py --gpus N --steps K --warmup W          # this implementation (libfav_b200.so, sm_100a)
   python bench.py --impl reference --gpus N ...           # the reference's CPU nn path (oracle port) on host cores
+  python bench.py ... --dump-outputs DIR                  # also write the last timed step's stylized frame to DIR
 
 A "step" = ONE FRAME of the hot path: fused warp+mask+preprocess+concat -> 7-channel input -> stylization net ->
 deprocess (run_next_image, fast_artistic_video_core.lua:161-180), recurrent (frame i consumes stylized i-1).
@@ -240,12 +241,8 @@ def run_ours(args):
         dist.all_reduce(t, op=dist.ReduceOp.MAX)
         return float(t.item())
 
-    # Timed regions: each is EXACTLY K steps bracketed by barrier + synchronize; regions repeat until >= 1 s of device time
-    # has been measured (so that short driver runs still amortise pipeline fill and give the clock sampler samples) and the
-    # MEDIAN region is reported.
-    def n_regions(t_first):
-        return max(1, min(60, int(1.0 / max(t_first, 1e-4)) + 1))
-
+    # Timed regions: each figure is ONE region of exactly K steps bracketed by barrier + synchronize, so that --steps is the
+    # number of timed steps and the last step's inputs (the recurrent state included) are the same from run to run.
     sampler = ClockSampler(local)
     if rank == 0:
         sampler.start()
@@ -275,14 +272,11 @@ def run_ours(args):
         barrier()
         return max_over_ranks(e0.elapsed_time(e1) / 1e3), int(_lib.lib.fav_launch_count() - l0)
 
-    t_first, launches = region_dev(False)
-    regions = n_regions(t_first)
-    t_list = sorted([t_first] + [region_dev(False)[0] for _ in range(regions - 1)])
-    t_dev = t_list[len(t_list) // 2]
+    t_dev, launches = region_dev(False)
+    out_last = prev  # the stylized frame of the last timed step: what --dump-outputs writes
     checksum = float(prev.double().sum().item())
     value = world * K / t_dev
-    tf_list = sorted(region_dev(True)[0] for _ in range(regions))
-    t_full = tf_list[len(tf_list) // 2]
+    t_full = region_dev(True)[0]
     value_full = world * K / t_full
 
     # ---- (2) end to end through the host-buffer API ------------------------------------------------------------
@@ -308,8 +302,7 @@ def run_ours(args):
         barrier()
         return max_over_ranks(time.perf_counter() - t0), t_enq
 
-    e_list = sorted(region_e2e() for _ in range(regions))
-    t_e2e, t_enqueue = e_list[len(e_list) // 2]
+    t_e2e, t_enqueue = region_e2e()
     tw1 = time.time()
     clocks = sampler.stop(tw0, tw1) if rank == 0 else None
     gpu_ms_last = sess.last_gpu_ms()
@@ -411,8 +404,8 @@ def run_ours(args):
                       "parallelism": f"replicas x{world} (independent clips, no data-path collective)",
                       "precision": "outputs within 1e-3 of the fp64 oracle (measured ~1e-5, tests/test_gpu_net.py, "
                                    "tests/test_gpu_parity_large.py)",
-                      "timing": f"{regions} timed regions of exactly {K} steps each (barrier + synchronize on both sides, CUDA "
-                                "events, max over ranks); value / e2e = the MEDIAN region"},
+                      "timing": f"one timed region of exactly {K} steps per figure (barrier + synchronize on both sides, max "
+                                "over ranks); value / value_full: CUDA events, e2e: host clock"},
             "e2e": {"value": e2e, "unit": "frames/s", "h2d_bytes_per_step": h2d, "d2h_bytes_per_step": d2h,
                     "ms_per_step": 1e3 * t_e2e / K, "host_enqueue_ms_per_step": 1e3 * t_enqueue / K,
                     "gpu_ms_last_frame": gpu_ms_last,
@@ -474,6 +467,9 @@ def run_ours(args):
         print(json.dumps(line), flush=True)
         if world > 1:
             os.dup2(2, 1)
+        if args.dump_outputs:
+            os.makedirs(args.dump_outputs, exist_ok=True)
+            np.save(os.path.join(args.dump_outputs, "stylized_frame.npy"), out_last.cpu().numpy())
     if world > 1:
         dist.destroy_process_group()
 
@@ -660,7 +656,12 @@ def main():
                          "the GPU; default) or decoded fp32 tensors")
     ap.add_argument("--arch", default="default", choices=list(ARCHS),
                     help="default = train_video.lua:21 (u64,u32); paper = README.md:256 (U2,c3s1-64,U2)")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write the stylized frame of the last timed step (rank 0) as "
+                         "DIR/stylized_frame.npy (float32, 3xHxW); the inputs are the same from run to run")
     args = ap.parse_args()
+    if args.dump_outputs and (args.impl != "ours" or args.config != "cfg2"):
+        ap.error("--dump-outputs applies to the default workload (--impl ours --config cfg2)")
     if args.warmup < 3:
         args.warmup = 3
     if args.impl == "reference":

@@ -1,7 +1,7 @@
 """The oracle is pinned before it is trusted (CPU only):
   * checkConsistency / computeCorners restatement == the reference's own consistencyChecker binary, bit for bit,
-    on the committed golden masks (tests/golden/consistency_*.npz, written by oracle/_ref) and, when the binary is
-    present, on fresh runs;
+    on the committed golden masks (tests/golden/consistency_*.npz, written by oracle/_ref), the frame passed in
+    memory and through a P6 file;
   * the warp restatement is cross-checked against torch grid_sample (independent implementation of per-corner
     zero fill), min_filter against F.max_pool2d, pre/deprocess against the Lua formula;
   * the torch net oracle reproduces its committed fp64 outputs and agrees fp32 vs fp64.
@@ -37,19 +37,21 @@ def test_consistency_oracle_equals_reference_binary_golden(case):
         assert (ref3 != ref4).sum() > 0  # the structure term is actually exercised
 
 
-@pytest.mark.skipif(not os.path.exists(pyoracle.REF_CHECKER), reason="oracle/_ref not built")
 def test_consistency_oracle_equals_reference_binary_live(tmp_path):
+    """The frame goes through a P6 file and read_ppm_planes, as the binary reads it; the binary's masks on these files
+    are tests/golden/consistency_72x88.npz (make_golden.py)."""
     H, W = 72, 88
+    g = np.load(os.path.join(GOLD, f"consistency_{H}x{W}.npz"))
+    ref3 = np.unpackbits(g["ref3"])[: H * W].reshape(H, W).astype(np.uint8) * 255
+    ref4 = np.unpackbits(g["ref4"])[: H * W].reshape(H, W).astype(np.uint8) * 255
     bw, fw, fr, _ = make_golden.consistency_inputs(H, W, 5, 0.5, 11)
     d = str(tmp_path)
-    synth.write_flo(d + "/bw.flo", bw); synth.write_flo(d + "/fw.flo", fw); synth.write_ppm(d + "/f.ppm", fr)
-    pyoracle.run_ref_checker(d + "/bw.flo", d + "/fw.flo", d + "/r3.pgm")
-    pyoracle.run_ref_checker(d + "/bw.flo", d + "/fw.flo", d + "/r4.pgm", d + "/f.ppm")
+    synth.write_ppm(d + "/f.ppm", fr)
     from fav_b200.consistencyChecker import read_ppm_planes
 
     img = read_ppm_planes(d + "/f.ppm")
-    assert np.array_equal(pyoracle.consistency(bw, fw), synth.read_pgm(d + "/r3.pgm"))
-    assert np.array_equal(pyoracle.consistency(bw, fw, img), synth.read_pgm(d + "/r4.pgm"))
+    assert np.array_equal(pyoracle.consistency(bw, fw), ref3)
+    assert np.array_equal(pyoracle.consistency(bw, fw, img), ref4)
 
 
 def test_warp_oracle_reproduces_reference_kernel_vectors():
